@@ -1,10 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- QPS at recall@10 >= 0.95, IVF-PQ d=128, 1B synthetic vectors, 8 shards.
 
-Contract (see the task statement): `python bench.py --gpus N --steps K --warmup W` prints ONE
-JSON line from rank 0.  A "step" is one pass of the hot path (IndexClient.search fan-out ->
-coarse quantizer -> PQ table -> inverted-list scan -> cross-shard merge) over one batch of
-`--batch` synthetic queries.  N>1 is launched by torchrun (one rank per GPU, NCCL).
+Usage: `python bench.py --gpus N --steps K --warmup W` prints ONE JSON line from rank 0.  A
+"step" is one pass of the hot path (IndexClient.search fan-out -> coarse quantizer -> PQ table ->
+inverted-list scan -> cross-shard merge) over one batch of `--batch` synthetic queries; every
+timed region runs K steps after W warm-up steps.  N>1 is launched by torchrun (one rank per GPU,
+NCCL).  `--dump-outputs DIR` writes what the last timed step returned (see dump_outputs), so
+that two builds can be compared output for output on the same seeded inputs.
 
 Workload (BASELINE.json configs[4], SURVEY.md 8d): N vectors, d=128, 8 shards (row block b of
 50 000 rows -> shard b mod 8, mimicking the client's round-robin), every shard its own IVF-PQ
@@ -166,6 +168,25 @@ class GroundTruth:
             dist.all_reduce(self.count)
         self.certified = self.count <= self.expected
         return int((~self.certified).sum().item())
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, D, I):
+    """One step's answer -- D [nq,k] float32 distances, I [nq,k] int64 row ids -- as
+    out_dir/distances.npy (float32) and out_dir/ids.npy (float64, exact for ids < 2**53), with the
+    query rows they belong to in out_dir/rows.npy.  Above DUMP_BYTES a fixed, seeded sample of the
+    query rows is kept."""
+    nq, k = D.shape
+    per_row = k * (4 + 8) + 8
+    rows = np.arange(nq)
+    if nq * per_row > DUMP_BYTES:
+        rows = np.sort(np.random.RandomState(0).choice(nq, DUMP_BYTES // per_row, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "distances.npy"), np.asarray(D, dtype=np.float32)[rows])
+    np.save(os.path.join(out_dir, "ids.npy"), np.asarray(I, dtype=np.float64)[rows])
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 def recall_at_k(I, gt, ok=None):
@@ -340,7 +361,12 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=2.0, help="minimum CPU time of one timed CPU sample")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the query-batch sweep 1/8/64/512/4096")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the answer of the last timed step into DIR (.npy)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the answer of the GPU path (--impl b200)")
 
     import torch
 
@@ -506,7 +532,8 @@ def main():
         return [xq.repeat((b // args.nq_pool) + 1, 1)[:b].contiguous()]
 
     def timed(batches_, steps, warmup, host=False):
-        """K steps bracketed by device events on EVERY rank (plane.timer_*), max over ranks"""
+        """K steps bracketed by device events on EVERY rank (plane.timer_*), max over ranks.
+        Returns (ms, what the last step returned)."""
         host_batches = [b.cpu().numpy() for b in batches_] if host else None
         run = (lambda i: client.search(host_batches[i % len(batches_)], K, "bench")) if host else \
               (lambda i: search_dev(batches_[i % len(batches_)]))
@@ -515,8 +542,8 @@ def main():
         torch.cuda.synchronize()
         plane.timer_start()
         for it in range(steps):
-            run(it)
-        return plane.timer_stop()
+            last = run(it)
+        return plane.timer_stop(), last
 
     B = args.batch
     batches = batches_of(B)
@@ -533,9 +560,12 @@ def main():
     clocks.start()
     launches0 = engine.launch_count()
     torch.cuda.profiler.start()   # for `ncu --profile-from-start off`; a no-op otherwise
-    ms = timed(batches, args.steps, args.warmup)
+    ms, (D_last, I_last) = timed(batches, args.steps, args.warmup)
     torch.cuda.profiler.stop()
     launches = engine.launch_count() - launches0
+    if args.dump_outputs:
+        # copied now: later searches may reuse the plane's result buffers
+        dump_outputs(args.dump_outputs, D_last.cpu().numpy(), I_last.cpu().numpy())
     scan_ms, scan_launches = 0.0, 0
     for s in shards:
         m, n = s.profile_read(reset=True)
@@ -549,7 +579,7 @@ def main():
 
     # e2e: IndexClient.search with HOST buffers -- pinned staging, H2D, the collective, one D2H,
     # integer metadata rows -- i.e. the call a user of the reference makes
-    ms_e2e = timed(batches, args.steps, args.warmup, host=True)
+    ms_e2e, _ = timed(batches, args.steps, args.warmup, host=True)
     clk = clocks.stop()
     qps_e2e = args.steps * B / (ms_e2e / 1e3)
     log(f"e2e done: {ms_e2e / args.steps:.3f} ms/step")
@@ -575,11 +605,10 @@ def main():
     if not args.no_sweep:
         for b in (1, 8, 64, 512, 4096):
             bb = batches_of(b)
-            st_ = max(args.steps, 100 if b <= 64 else args.steps)
-            t = timed(bb, st_, args.warmup)
-            sweep[str(b)] = st_ * b / (t / 1e3)
-            t = timed(bb, st_, args.warmup, host=True)
-            sweep_e2e[str(b)] = st_ * b / (t / 1e3)
+            t, _ = timed(bb, args.steps, args.warmup)
+            sweep[str(b)] = args.steps * b / (t / 1e3)
+            t, _ = timed(bb, args.steps, args.warmup, host=True)
+            sweep_e2e[str(b)] = args.steps * b / (t / 1e3)
         log(f"sweep: {sweep}")
 
     # roofline of the dominant kernel: algorithmic bytes = ndis * code_bytes (SURVEY 8d)

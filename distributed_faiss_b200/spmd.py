@@ -509,6 +509,10 @@ class SearchPlane:
                     self._run_search(h, index_id, blob, None)
 
     def stop(self):
+        global _current_plane
+        with _plane_lock:   # an IndexClient created from now on must not attach to a stopped plane
+            if _current_plane is self:
+                _current_plane = None
         if self.rank == 0 and self.world > 1:
             with self._lock, self._stream_ctx():
                 self._send_header([OP_STOP])

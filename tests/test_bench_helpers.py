@@ -45,3 +45,24 @@ def test_recall_at_k():
     gt2 = gt.clone()
     gt2[1, -2:] = -1                                   # a group with only K-2 members
     assert abs(bench.recall_at_k(gt.clone(), gt2) - 1.0) < 1e-6
+
+
+def test_dump_outputs(tmp_path, monkeypatch):
+    """--dump-outputs: float32 distances, float64 ids, every row while it fits; above the size
+    limit the same seeded sample of rows every time."""
+    rs = np.random.RandomState(0)
+    D = rs.rand(100, bench.K).astype(np.float32)
+    I = rs.randint(0, 1 << 40, size=(100, bench.K)).astype(np.int64)
+    bench.dump_outputs(str(tmp_path / "all"), D, I)
+    d, i, r = (np.load(tmp_path / "all" / f) for f in ("distances.npy", "ids.npy", "rows.npy"))
+    assert d.dtype == np.float32 and i.dtype == np.float64 and r.dtype == np.float64
+    assert np.array_equal(d, D) and np.array_equal(i.astype(np.int64), I) and np.array_equal(r, np.arange(100))
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 30 * (bench.K * 12 + 8))
+    for name in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / name), D, I)
+    ra, rb = np.load(tmp_path / "a" / "rows.npy"), np.load(tmp_path / "b" / "rows.npy")
+    assert len(ra) == 30 and np.array_equal(ra, rb) and (np.diff(ra) > 0).all()
+    rows = ra.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "distances.npy"), D[rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "ids.npy").astype(np.int64), I[rows])

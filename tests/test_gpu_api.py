@@ -315,8 +315,12 @@ def test_index_client_collective_plane_equals_socket_fanout():
         assert np.array_equal(D2, Dp if False else D2) and D2.shape == (33, 7)
     finally:
         client.close()
+        plane.stop()
         for s in servers:
             s.stop()
+    # a client created later in this process (another cluster with as many servers) must not attach
+    from distributed_faiss_b200 import spmd
+    assert spmd.current_plane() is None
 
 
 def test_async_trained_shard_stays_on_its_device():
