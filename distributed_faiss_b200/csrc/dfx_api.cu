@@ -74,12 +74,18 @@ int dfx_create(const dfx_cfg* cfg, dfx_index** out) {
         DFX_REQUIRE(cfg->d % 4 == 0, "IVF indexes need a dimension that is a multiple of 4");
     }
     if (cfg->kind == DFX_IVF_PQ) {
-        DFX_REQUIRE(cfg->pq_nbits == 8, "IVF-PQ: only 8 bits per sub-quantizer are supported");
+        DFX_REQUIRE(cfg->pq_nbits == 8 || cfg->pq_nbits == 4,
+                    "IVF-PQ: bits per sub-quantizer must be 4 or 8, got " + std::to_string(cfg->pq_nbits));
         DFX_REQUIRE(cfg->pq_m >= 4 && cfg->pq_m % 4 == 0 && cfg->d % cfg->pq_m == 0,
                     "IVF-PQ: the number of sub-quantizers must be a multiple of 4 that divides d");
         DFX_REQUIRE(cfg->pq_m <= 64, "IVF-PQ: at most 64 sub-quantizers are supported");
+        // 4-bit rows are M / 2 bytes; M % 8 == 0 keeps them whole 4-byte words (finalize, scan loads)
+        DFX_REQUIRE(cfg->pq_nbits == 8 || cfg->pq_m % 8 == 0,
+                    "IVF-PQ with 4-bit codes: the number of sub-quantizers must be a multiple of 8, got " +
+                        std::to_string(cfg->pq_m));
         idx->M = cfg->pq_m;
-        idx->ksub = 256;
+        idx->nbits = cfg->pq_nbits;
+        idx->ksub = 1 << cfg->pq_nbits;
         idx->dsub = cfg->d / cfg->pq_m;
     }
     DeviceGuard g(cfg->device);

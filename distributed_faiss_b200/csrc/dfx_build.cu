@@ -76,22 +76,13 @@ __global__ void split_cluster_kernel(float* cent, int d, int empty, int big) {
     }
 }
 
-// PQ encode: grid (ceil(n/256), M); code_m = argmin_j l2_seq(r_m, P[m][j]), ties -> smaller j.
-// The residual sub-vector lives in registers (DS = dsub when it is one of the common sizes).
+// PQ encode: grid (ceil(n/256), row bytes); code_m = argmin_j l2_seq(r_m, P[m][j]), ties -> smaller
+// j.  A thread writes one whole byte of a row: one code at 8 bits, the two codes that share the
+// byte at 4 bits (so no two threads write the same byte).  The residual sub-vector lives in
+// registers (DS = dsub when it is one of the common sizes).
 template <int DS>
-__global__ void __launch_bounds__(256)
-pq_encode_kernel(const float* __restrict__ x, const float* __restrict__ cent,
-                 const int32_t* __restrict__ assign, int64_t n, int d, int M, int ksub, int dsub,
-                 const float* __restrict__ codebooks, uint8_t* __restrict__ codes) {
-    DFX_DYN_SMEM0(float, s_cb);  // [ksub][dsub]
-    const int m = blockIdx.y;
-    for (int i = threadIdx.x; i < ksub * dsub; i += blockDim.x)
-        s_cb[i] = codebooks[(size_t)m * ksub * dsub + i];
-    __syncthreads();
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float* xi = x + i * d + m * dsub;
-    const float* c = cent + (size_t)assign[i] * d + m * dsub;
+__device__ __forceinline__ int pq_encode_one(const float* __restrict__ xi, const float* __restrict__ c,
+                                             const float* __restrict__ s_cb, int ksub, int dsub) {
     float best = FLT_MAX;
     int bj = 0;
     if (DS > 0) {
@@ -123,13 +114,38 @@ pq_encode_kernel(const float* __restrict__ x, const float* __restrict__ cent,
             }
         }
     }
-    codes[i * M + m] = (uint8_t)bj;
+    return bj;
+}
+
+template <int DS>
+__global__ void __launch_bounds__(256)
+pq_encode_kernel(const float* __restrict__ x, const float* __restrict__ cent,
+                 const int32_t* __restrict__ assign, int64_t n, int d, int M, int ksub, int dsub, int nbits,
+                 const float* __restrict__ codebooks, uint8_t* __restrict__ codes) {
+    DFX_DYN_SMEM0(float, s_cb);  // [per][ksub][dsub]: the codebooks of the byte's sub-quantizers
+    const int per = 8 / nbits;   // codes per byte
+    const int b = blockIdx.y, m0 = b * per;
+    for (int i = threadIdx.x; i < per * ksub * dsub; i += blockDim.x)
+        s_cb[i] = codebooks[(size_t)m0 * ksub * dsub + i];
+    __syncthreads();
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float* xi = x + i * d + m0 * dsub;
+    const float* c = cent + (size_t)assign[i] * d + m0 * dsub;
+    const int c0 = pq_encode_one<DS>(xi, c, s_cb, ksub, dsub);
+    const int64_t rb = (int64_t)M * nbits / 8;
+    if (nbits == 8) {
+        codes[i * rb + b] = (uint8_t)c0;
+    } else {
+        const int c1 = pq_encode_one<DS>(xi + dsub, c + dsub, s_cb + ksub * dsub, ksub, dsub);
+        codes[i * rb + b] = dfx_pq4_byte(c0, c1);
+    }
 }
 
 // tvals[i] = sum_m ( |p_m|^2 + 2 <c_m, p_m> ), sequential in m (oracle orc_pq_tvals)
 __global__ void pq_tvals_kernel(const uint8_t* __restrict__ codes, const int32_t* __restrict__ list_of,
                                 const int64_t* __restrict__ list_off, int64_t nlist, int64_t n, int d,
-                                int M, int ksub, int dsub, const float* __restrict__ codebooks,
+                                int M, int ksub, int dsub, int nbits, const float* __restrict__ codebooks,
                                 const float* __restrict__ cent, float* __restrict__ tvals) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -145,9 +161,10 @@ __global__ void pq_tvals_kernel(const uint8_t* __restrict__ codes, const int32_t
         l = lo;
     }
     const float* c = cent + (size_t)l * d;
+    const uint8_t* row = codes + i * ((int64_t)M * nbits / 8);
     float t = 0.f;
     for (int m = 0; m < M; m++) {
-        const float* p = codebooks + ((size_t)m * ksub + codes[i * M + m]) * dsub;
+        const float* p = codebooks + ((size_t)m * ksub + dfx_pq_code(row, m, nbits)) * dsub;
         float ipcp = 0.f, ippp = 0.f;
         for (int tt = 0; tt < dsub; tt++) ipcp = __fmaf_rn(c[m * dsub + tt], p[tt], ipcp);
         for (int tt = 0; tt < dsub; tt++) ippp = __fmaf_rn(p[tt], p[tt], ippp);
@@ -410,13 +427,14 @@ void dfx_add_impl(dfx_index* idx, int64_t n, const float* d_x, cudaStream_t st) 
     if (kind == DFX_IVF_FLAT) {
         DFX_CUDA(cudaMemcpyAsync(prow, d_x, (size_t)n * rb, cudaMemcpyDeviceToDevice, st));
     } else if (kind == DFX_IVF_PQ) {
-        const int M = idx->M, ksub = idx->ksub, dsub = idx->dsub;
-        dim3 grid(blocks_for(n, 256), (unsigned)M);
+        const int M = idx->M, ksub = idx->ksub, dsub = idx->dsub, nbits = idx->nbits;
+        dim3 grid(blocks_for(n, 256), (unsigned)rb);  // one thread per (vector, row byte)
+        const size_t cb_smem = (size_t)(8 / nbits) * ksub * dsub * 4;
 #define DFX_PQ_ENCODE(DS)                                                                       \
     do {                                                                                        \
         auto kern = pq_encode_kernel<DS>;                                                       \
-        DFX_LAUNCH(kern, grid, 256, (size_t)ksub * dsub * 4, st, d_x, idx->centroids.as<float>(), \
-                   plist, n, d, M, ksub, dsub, idx->codebooks.as<float>(), (uint8_t*)prow);     \
+        DFX_LAUNCH(kern, grid, 256, cb_smem, st, d_x, idx->centroids.as<float>(),               \
+                   plist, n, d, M, ksub, dsub, nbits, idx->codebooks.as<float>(), (uint8_t*)prow); \
     } while (0)
         if (dsub == 2) DFX_PQ_ENCODE(2);
         else if (dsub == 4) DFX_PQ_ENCODE(4);
@@ -425,7 +443,7 @@ void dfx_add_impl(dfx_index* idx, int64_t n, const float* d_x, cudaStream_t st) 
         else DFX_PQ_ENCODE(0);
 #undef DFX_PQ_ENCODE
         DFX_LAUNCH(pq_tvals_kernel, blocks_for(n, 128), 128, 0, st, (const uint8_t*)prow, plist,
-                   (const int64_t*)nullptr, nlist, n, d, M, ksub, dsub, idx->codebooks.as<float>(),
+                   (const int64_t*)nullptr, nlist, n, d, M, ksub, dsub, nbits, idx->codebooks.as<float>(),
                    idx->centroids.as<float>(), idx->p_tvals.as<float>() + idx->n_pending);
     } else {  // IVF_SQ16
         DFX_LAUNCH(sq_encode_kernel, blocks_for(n * d, 256), 256, 0, st, d_x, idx->centroids.as<float>(),
@@ -440,7 +458,7 @@ void dfx_compute_tvals_sorted(dfx_index* idx, cudaStream_t st) {
     if (n == 0) return;
     DFX_LAUNCH(pq_tvals_kernel, blocks_for(n, 128), 128, 0, st, idx->payload.as<uint8_t>(),
                (const int32_t*)nullptr, idx->list_off.as<int64_t>(), idx->cfg.nlist, n, idx->cfg.d,
-               idx->M, idx->ksub, idx->dsub, idx->codebooks.as<float>(), idx->centroids.as<float>(),
+               idx->M, idx->ksub, idx->dsub, idx->nbits, idx->codebooks.as<float>(), idx->centroids.as<float>(),
                idx->tvals.as<float>());
 }
 
@@ -519,7 +537,7 @@ void dfx_finalize_impl(dfx_index* idx, cudaStream_t st) {
     idx->n_sorted = n;
     idx->n_pending = 0;
     idx->inv_valid = false;
-    dfx_pq_rm_to_il(idx, st);  // IVF-PQ, M == 32: interleaved blocks for the scan (no-op otherwise)
+    dfx_pq_rm_to_il(idx, st);  // IVF-PQ 32 x 8 / 64 x 4 bit: interleaved blocks for the scan (no-op otherwise)
 }
 
 // ------------------------------------------------------------------ reconstruct
@@ -529,8 +547,9 @@ __global__ void invert_ids_kernel(const int32_t* __restrict__ ids, int64_t n, in
 }
 
 // il != 0 (IVF-PQ interleaved, il = block layout 1 or 2): `inv` holds padded block positions and
-// codes are read from the interleaved blocks (dfx_il_byte_of(il, pos%32, m) of block pos/32)
-__global__ void reconstruct_kernel(int kind, int d, int M, int ksub, int dsub, int64_t ntotal,
+// codes are read from the interleaved blocks (dfx_il_byte_of(il, pos%32, m & 31) of block pos/32;
+// at 4 bits that byte is the pair of columns m & 31, dfx_il2_pair_code)
+__global__ void reconstruct_kernel(int kind, int d, int M, int ksub, int dsub, int nbits, int64_t ntotal,
                                    int64_t nlist, const int64_t* __restrict__ want,
                                    const int32_t* __restrict__ inv, const void* __restrict__ rows,
                                    const int64_t* __restrict__ list_off, const float* __restrict__ cent,
@@ -570,8 +589,12 @@ __global__ void reconstruct_kernel(int kind, int d, int M, int ksub, int dsub, i
         } else {
             int m = k / dsub;
             int code;
-            if (il) code = reinterpret_cast<const uint8_t*>(rows)[(pos >> 5) * 1024 + dfx_il_byte_of(il, (int)(pos & 31), m)];
-            else code = reinterpret_cast<const uint8_t*>(rows)[pos * M + m];
+            if (il) {
+                const uint8_t b = reinterpret_cast<const uint8_t*>(rows)[(pos >> 5) * 1024 + dfx_il_byte_of(il, (int)(pos & 31), m & 31)];
+                code = (nbits == 8) ? (int)b : dfx_il2_pair_code(b, m);
+            } else {
+                code = dfx_pq_code(reinterpret_cast<const uint8_t*>(rows) + pos * ((int64_t)M * nbits / 8), m, nbits);
+            }
             v = cent[(size_t)l * d + k] + codebooks[((size_t)m * ksub + code) * dsub + (k - m * dsub)];
         }
         out[r * d + k] = v;
@@ -593,7 +616,7 @@ void dfx_reconstruct_impl(dfx_index* idx, int64_t n, const int64_t* d_ids, float
         idx->inv_valid = true;
     }
     DFX_LAUNCH(reconstruct_kernel, (unsigned)n, 128, 0, st, idx->cfg.kind, idx->cfg.d, idx->M, idx->ksub,
-               idx->dsub, nt, idx->cfg.nlist, d_ids, idx->inv.as<int32_t>(),
+               idx->dsub, idx->nbits, nt, idx->cfg.nlist, d_ids, idx->inv.as<int32_t>(),
                il ? (const void*)idx->il_codes.p : (const void*)idx->payload.p, idx->list_off.as<int64_t>(),
                idx->centroids.as<float>(), idx->codebooks.as<float>(), il, idx->blk_off.as<int64_t>(), d_out, tag);
 }

@@ -10,6 +10,7 @@
 struct dfx_index {
     dfx_cfg cfg{};
     int M = 0, ksub = 0, dsub = 0;
+    int nbits = 8;  // IVF-PQ bits per sub-quantizer code (4 or 8); ksub = 1 << nbits
     int64_t nprobe = 1;  // faiss default (index.py:47 copies it back into cfg for knnlm)
     bool trained = false;
 
@@ -36,8 +37,9 @@ struct dfx_index {
     int max_points_per_centroid = 256;  // faiss Clustering default
     uint64_t train_seed = 1234;       // faiss Clustering default seed
 
-    // IVF-PQ, M == 32: block-interleaved storage for the lane-per-vector scan (dfx_scan_il2.cu,
-    // layout dfx_il2_byte).  While `il` is set the row-major payload/tvals/ids are released.
+    // IVF-PQ, M == 32 x 8 bit or M == 64 x 4 bit: block-interleaved storage for the lane-per-vector
+    // scan (dfx_scan_il2.cu, layout dfx_il2_byte / dfx_il2_pair).  While `il` is set the row-major
+    // payload/tvals/ids are released.
     bool il = false, il_enabled = true;
     DevBuf il_codes, il_tvals, il_ids, blk_off;
     int64_t nblk = 0;
@@ -125,7 +127,7 @@ struct dfx_index {
         switch (cfg.kind) {
             case DFX_FLAT:
             case DFX_IVF_FLAT: return (size_t)cfg.d * 4;
-            case DFX_IVF_PQ: return (size_t)M;
+            case DFX_IVF_PQ: return (size_t)M * nbits / 8;
             case DFX_IVF_SQ16: return (size_t)cfg.d * 2;
         }
         return 0;
@@ -162,7 +164,8 @@ void dfx_stats_impl(dfx_index* idx, int64_t* ndis, cudaStream_t st);
 void dfx_launch_select_comp(const uint64_t* comp, int64_t nrows, int n, int64_t ld, int k, int32_t* keys,
                             cudaStream_t st);
 
-// Interleaved IVF-PQ block (M == 32): 32 vectors x 32 codes = 1 KB, one lane per vector.
+// Interleaved IVF-PQ block (M == 32 x 8 bit; M == 64 x 4 bit stores code pairs, dfx_il2_pair below):
+// 32 vectors x 32 bytes = 1 KB, one lane per vector.
 // Lane v of the scanning warp owns vector v of
 // the block and walks its 32 subquantizers in the rotated order m = (t + v) & 31, t = 0..31, so
 // that at every step the 32 lanes read 32 different table columns (bank == column).  Byte t of
@@ -176,6 +179,28 @@ __host__ __device__ __forceinline__ int dfx_il2_byte(int v, int m) {
 // (the `layout` argument of the C-ABI probe dfx_debug_il_byte is kept for compatibility; there is
 // one block layout)
 __host__ __device__ __forceinline__ int dfx_il_byte_of(int /*layout*/, int v, int m) { return dfx_il2_byte(v, m); }
+
+// ---- PQ code format.  Every reader and writer of PQ codes goes through the helpers below.
+// Row-major (exchange) form, faiss bit order (PQEncoderGeneric, LSB first): a row is M * nbits / 8
+// bytes; at nbits = 8 byte m is code m, at nbits = 4 byte m >> 1 holds code m in its low nibble
+// when m is even and in its high nibble when m is odd.
+__host__ __device__ __forceinline__ int dfx_pq_code(const uint8_t* row, int m, int nbits) {
+    return nbits == 8 ? (int)row[m] : (int)((row[m >> 1] >> ((m & 1) * 4)) & 15u);
+}
+// byte b of a 4-bit row from its two codes (sub-quantizers 2b and 2b + 1)
+__host__ __device__ __forceinline__ uint8_t dfx_pq4_byte(int c_even, int c_odd) {
+    return (uint8_t)(c_even | (c_odd << 4));
+}
+// code u (0..7) of 4-byte word w of a 4-bit row (sub-quantizer 8w + u; the row is little endian)
+__host__ __device__ __forceinline__ int dfx_pq4_word_code(uint32_t word, int u) {
+    return (int)((word >> (4 * u)) & 15u);
+}
+// Blocks of the fused M = 64 x 4-bit scan: byte dfx_il2_byte(v, p), p < 32, holds the PAIR
+// c_p | c_{p+32} << 4 of vector v -- one byte per column of the pair table (dfx_scan_il2_dev.cuh),
+// so the block bytes, offsets and addressing are those of the M = 32 x 8-bit blocks.
+__host__ __device__ __forceinline__ uint8_t dfx_il2_pair(int c_p, int c_p32) { return (uint8_t)(c_p | (c_p32 << 4)); }
+// code of sub-quantizer m < 64 in the pair byte of column m & 31
+__host__ __device__ __forceinline__ int dfx_il2_pair_code(uint8_t pair, int m) { return (int)((pair >> ((m >> 5) * 4)) & 15u); }
 
 // ---- dfx_scan_il.cu
 bool dfx_il_wanted(const dfx_index* idx);

@@ -5,9 +5,9 @@
 #include "dfx_ptx.cuh"
 
 // =====================================================================================
-// K3 (row-major scan, M != 32 or interleaving switched off): lut[q][m][j] = -2 * ip_seq(q_m, P[m][j]);
-// dis0[q][p] = warp-dot ||q - c||^2.  (The M == 32 block scan builds its table in its own
-// prologue, dfx_scan_il2_dev.cuh.)
+// K3 (row-major scan: any other (M, nbits), or interleaving switched off): lut[q][m][j] =
+// -2 * ip_seq(q_m, P[m][j]), j < ksub (256 or 16); dis0[q][p] = warp-dot ||q - c||^2.  (The block
+// scan of M == 32 x 8 / M == 64 x 4 bit builds its table in its own prologue, dfx_scan_il2_dev.cuh.)
 // =====================================================================================
 __global__ void __launch_bounds__(256)
 pq_prep_kernel(const float* __restrict__ Q, int d, int M, int ksub, int dsub,

@@ -1,9 +1,11 @@
-// dfx_scan_il.cu -- layout conversion drivers of the block-interleaved IVF-PQ storage (M == 32).
+// dfx_scan_il.cu -- layout conversion drivers of the block-interleaved IVF-PQ storage (M == 32 x 8 bit
+// and M == 64 x 4 bit).
 // Kernels: dfx_scan_il_dev.cuh; the scan itself: dfx_scan_il2.cu.
 #include "dfx_scan_il_dev.cuh"
 
 bool dfx_il_wanted(const dfx_index* idx) {
-    return idx->cfg.kind == DFX_IVF_PQ && idx->M == 32 && idx->il_enabled;
+    return idx->cfg.kind == DFX_IVF_PQ && idx->il_enabled &&
+           ((idx->M == 32 && idx->nbits == 8) || (idx->M == 64 && idx->nbits == 4));
 }
 
 // payload/tvals/ids (row-major, list-sorted) -> il_* ; frees the row-major arrays
@@ -23,7 +25,7 @@ void dfx_pq_rm_to_il(dfx_index* idx, cudaStream_t st) {
     idx->il_ids.reserve((size_t)std::max<int64_t>(nblk, 1) * 32 * 4);
     if (nblk > 0)
         DFX_LAUNCH(pq_rm_to_il_kernel, (unsigned)nblk, 256, 0, st, idx->list_off.as<int64_t>(),
-                   idx->blk_off.as<int64_t>(), nlist, idx->payload.as<uint8_t>(), idx->tvals.as<float>(),
+                   idx->blk_off.as<int64_t>(), nlist, idx->nbits, idx->payload.as<uint8_t>(), idx->tvals.as<float>(),
                    idx->ids.as<int32_t>(), idx->il_codes.as<uint8_t>(), idx->il_tvals.as<float>(),
                    idx->il_ids.as<int32_t>());
     DFX_CUDA(cudaStreamSynchronize(st));  // h_blk is on the stack of this call
@@ -39,12 +41,12 @@ void dfx_pq_rm_to_il(dfx_index* idx, cudaStream_t st) {
 void dfx_pq_il_to_rm(dfx_index* idx, cudaStream_t st) {
     if (!idx->il) return;
     const int64_t n = idx->n_sorted;
-    idx->payload.reserve((size_t)std::max<int64_t>(n, 1) * 32);
+    idx->payload.reserve((size_t)std::max<int64_t>(n, 1) * idx->row_bytes());
     idx->tvals.reserve((size_t)std::max<int64_t>(n, 1) * 4);
     idx->ids.reserve((size_t)std::max<int64_t>(n, 1) * 4);
     if (idx->nblk > 0)
         DFX_LAUNCH(pq_il_to_rm_kernel, (unsigned)idx->nblk, 256, 0, st, idx->list_off.as<int64_t>(),
-                   idx->blk_off.as<int64_t>(), idx->cfg.nlist, idx->il_codes.as<uint8_t>(),
+                   idx->blk_off.as<int64_t>(), idx->cfg.nlist, idx->nbits, idx->il_codes.as<uint8_t>(),
                    idx->il_tvals.as<float>(), idx->il_ids.as<int32_t>(), idx->payload.as<uint8_t>(),
                    idx->tvals.as<float>(), idx->ids.as<int32_t>());
     DFX_CUDA(cudaStreamSynchronize(st));

@@ -36,6 +36,11 @@
 //     memory (268 MB written + 268 MB read per 4096-query launch) and the K3 launch is gone.
 //   * A CTA that owns ALL probes of its query (ngroups == 1, the large-batch regime) writes the
 //     final (D, I) rows itself; the per-query reduction launch is skipped.
+//   * M = 64 x 4 bit (PQ4) runs the same main loop: block byte p of a vector is the pair
+//     c_p | c_{p+32} << 4 and the prologue builds the pair table T[b][p] = lut[p][b & 15] +
+//     lut[p+32][b >> 4] in place of the 8-bit table.  That sum is the first level (s[p] + s[p+32])
+//     of the oracle's M = 64 tree; its other five levels are the M = 32 tree the loop already
+//     reproduces, so the sums are bit-identical with 32 lookups per vector (DESIGN.md 4.2).
 #pragma once
 #include "dfx_internal.h"
 #include "dfx_topk.cuh"
@@ -95,10 +100,40 @@ __device__ __noinline__ Il2Flushed il2_flush(uint64_t kept, uint64_t* queue, int
     return r;
 }
 
+// Prologue of the M = 64 x 4-bit block scan (out of line: it keeps the main loop's register
+// allocation that of the 8-bit kernel).  (a) lut[m][j] = -2 * ip_seq(q_m, P[m][j]), m < 64,
+// j < 16, into s_l16 (the queue area, free until the scan starts; >= 4 KB for every k), stored
+// [j][m] so that (b) reads it conflict-free.  (b) the pair table T[b][p] = lut[p][b & 15] +
+// lut[p + 32][b >> 4] -- the first level of the oracle's M = 64 halving tree (s[p] + s[p + 32]);
+// b = pair byte of column p (dfx_il2_pair).  Row b is 64 floats wide with columns p and p + 32
+// equal, as in the 8-bit table.
+template <int THREADS>
+__device__ __noinline__ void il2_pair_table(float* s_lut, float* s_l16, const float* __restrict__ qrow,
+                                            const float* __restrict__ cbT, int dsub, int tid) {
+#pragma unroll 1
+    for (int e = tid; e < 16 * 64; e += THREADS) {  // e = j * 64 + m: cbT row e is P[m][j]
+        const int m = e & 63;
+        const float* pv = cbT + (size_t)e * dsub;
+        const float* qm = qrow + m * dsub;
+        float acc = 0.f;
+        for (int t = 0; t < dsub; t++) acc = __fmaf_rn(__ldg(qm + t), __ldg(pv + t), acc);
+        s_l16[e] = -2.f * acc;
+    }
+    __syncthreads();
+#pragma unroll 1
+    for (int e = tid; e < 256 * 32; e += THREADS) {
+        const int b = e >> 5, p = e & 31;
+        const float val = s_l16[(b & 15) * 64 + p] + s_l16[(b >> 4) * 64 + 32 + p];
+        s_lut[b * 64 + p] = val;
+        s_lut[b * 64 + 32 + p] = val;
+    }
+}
+
 // REG: k <= 32, register-resident top-k;  !REG: WarpTopK buffers in shared memory (any k)
-// Q [nq][d] queries; cbT: transposed codebook PT[j][m][dsub]; cent [nlist][d]; d = 32 * dsub.
+// PQ4: M = 64 x 4 bit (pair table, blocks of pair bytes); else M = 32 x 8 bit.
+// Q [nq][d] queries; cbT: transposed codebook PT[j][m][dsub]; cent [nlist][d]; d = M * dsub.
 // outD / outI != nullptr (requires ngroups == 1): final faiss-style rows are written directly.
-template <bool REG, int THREADS, int MINB>
+template <bool REG, int THREADS, int MINB, bool PQ4>
 __global__ void __launch_bounds__(THREADS, MINB)
 scan_pq_il2_kernel(const float* __restrict__ Q, const float* __restrict__ cbT, const float* __restrict__ cent, int d,
                    int dsub, const int32_t* __restrict__ keys, int nprobe, int G, int ngroups,
@@ -134,7 +169,9 @@ scan_pq_il2_kernel(const float* __restrict__ Q, const float* __restrict__ cbT, c
     }
     // ---- K3, part 1: the query's table, rows j = warp, warp + 8, ...; lane = subquantizer m.
     // seq-k order (oracle): acc = fma(q0, p0, 0), fma(q1, p1, acc), ...; entry = -2 * acc.
-    if (dsub == 4) {
+    if (PQ4) {
+        il2_pair_table<THREADS>(s_lut, reinterpret_cast<float*>(s_buf), qrow, cbT, dsub, tid);
+    } else if (dsub == 4) {
         const float4 qm = __ldg(reinterpret_cast<const float4*>(qrow) + lane);
         const float4* pt4 = reinterpret_cast<const float4*>(cbT);
 #pragma unroll 8

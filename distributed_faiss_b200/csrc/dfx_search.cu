@@ -198,7 +198,7 @@ scan_pq_kernel(const float* __restrict__ lut, const float* __restrict__ dis0,
                const int32_t* __restrict__ keys, int nprobe, int G, int ngroups,
                const int64_t* __restrict__ list_off, const uint8_t* __restrict__ codes,
                const float* __restrict__ tvals, const int32_t* __restrict__ ids, int Mrt, int ksub,
-               int k, int cap, uint64_t* __restrict__ part) {
+               int nbits, int k, int cap, uint64_t* __restrict__ part) {
     DFX_DYN_SMEM(unsigned char, smem_raw, 16);
     const int M = (MT > 0) ? MT : Mrt;
     float* s_lut = reinterpret_cast<float*>(smem_raw);
@@ -232,7 +232,21 @@ scan_pq_kernel(const float* __restrict__ lut, const float* __restrict__ dis0,
                 // table values of this vector, then the canonical halving tree (oracle pq_sum)
                 constexpr int P = (MT > 0) ? MT : 64;  // MT is a power of two when > 0
                 float val[P];
-                if (MT > 0 && (MT % 16) == 0) {
+                if (nbits == 4) {  // ksub = 16, rows of M / 2 bytes (M % 8 == 0): 8 codes per word
+                    const uint32_t* cp = reinterpret_cast<const uint32_t*>(codes + i * (int64_t)(M / 2));
+#pragma unroll
+                    for (int w = 0; w < (P + 7) / 8; w++) {
+                        const int m = w * 8;
+                        if (m < M) {
+                            const uint32_t c = __ldg(cp + w);
+#pragma unroll
+                            for (int u = 0; u < 8; u++) val[m + u] = s_lut[(m + u) * 16 + dfx_pq4_word_code(c, u)];
+                        } else {
+#pragma unroll
+                            for (int u = 0; u < 8; u++) val[m + u] = 0.f;
+                        }
+                    }
+                } else if (MT > 0 && (MT % 16) == 0) {
                     const uint4* cp = reinterpret_cast<const uint4*>(codes + i * (int64_t)M);
 #pragma unroll
                     for (int w4 = 0; w4 < MT / 16; w4++) {
@@ -722,7 +736,7 @@ void dfx_search_impl(dfx_index* idx, int64_t nq, const float* d_x, int64_t k64, 
 
         bool final_written = false;
         if (kind == DFX_IVF_PQ && idx->il) {
-            // M == 32: table build + exact |q-c|^2 + block scan in ONE kernel; with a single probe
+            // M == 32 x 8 / 64 x 4 bit: table build + exact |q-c|^2 + block scan in ONE kernel; with a single probe
             // group per query it also writes the final rows (dfx_scan_il2.cu)
             final_written = dfx_launch_scan_pq_il2(idx, xq, qc, keys, nprobe, G, ngroups, k, cap, part, d_D + q0 * k,
                                                    d_I + q0 * k, st);
@@ -744,7 +758,7 @@ void dfx_search_impl(dfx_index* idx, int64_t nq, const float* d_x, int64_t k64, 
         DFX_LAUNCH(kern, (unsigned)(qc * ngroups), 128, smem, st, idx->w_lut.as<float>(),        \
                    idx->w_dis0.as<float>(), keys, nprobe, G, ngroups, idx->list_off.as<int64_t>(), \
                    idx->payload.as<uint8_t>(), idx->tvals.as<float>(), idx->ids.as<int32_t>(), M, \
-                   ksub, k, cap, part);                                                          \
+                   ksub, idx->nbits, k, cap, part);                                              \
     } while (0)
             if (M == 32) DFX_SCAN_PQ(32);
             else if (M == 64) DFX_SCAN_PQ(64);

@@ -124,6 +124,7 @@ class GpuIndex:
         if self.kind != KIND_FLAT:
             self.quantizer = _Quantizer(self)
         self.pq_m = int(pq_m)
+        self.pq_nbits = int(pq_nbits)
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -299,9 +300,11 @@ class GpuIndex:
         else:
             st["coarse_metric"] = self.metric
         if self.kind == KIND_IVF_PQ:
-            st["M"], st["ksub"] = self.pq_m, 256
-            st["codebooks"] = self.get_array("codebooks").reshape(self.pq_m, 256, d // self.pq_m)
-            st["codes"] = self.get_array("codes").reshape(-1, self.pq_m)
+            # codes: M * nbits / 8 bytes per vector in faiss bit order (include/dfx.h "codes")
+            ksub = 1 << self.pq_nbits
+            st["M"], st["ksub"] = self.pq_m, ksub
+            st["codebooks"] = self.get_array("codebooks").reshape(self.pq_m, ksub, d // self.pq_m)
+            st["codes"] = self.get_array("codes").reshape(-1, self.pq_m * self.pq_nbits // 8)
             st["tvals"] = self.get_array("tvals")
         if self.kind == KIND_IVF_SQ16:
             st["codes16"] = self.get_array("codes16").reshape(-1, d)

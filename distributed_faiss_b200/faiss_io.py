@@ -23,7 +23,10 @@ Layout (little endian, no padding; `vec<T>` = u64 count + raw elements):
              every non-empty list: codes (size * code_size bytes), ids (size * i64)
   IVFFlat  : "IwFl", ivf hdr, invlists (code = raw f32 vector)
   IVFPQ    : "IwPQ", ivf hdr, u8 by_residual, u64 code_size, PQ (u64 d, u64 M, u64 nbits,
-             vec<f32> centroids [M][ksub][dsub]), invlists (code = M bytes)
+             vec<f32> centroids [M][ksub][dsub]), invlists (code = M * nbits / 8 bytes; nbits 8
+             or 4, 4-bit codes packed LSB first: code m in the low nibble of byte m >> 1 when m is
+             even, in the high nibble when odd -- faiss PQEncoderGeneric order, which is also the
+             order of the engine state dict)
   IVFSQ    : "IwSq", ivf hdr, SQ (i32 qtype = 4 (fp16), i32 rangestat, f32 rangestat_arg, u64 d,
              u64 code_size, vec<f32> trained (empty)), u64 code_size, u8 by_residual, invlists
              (code = d little-endian fp16 of the residual)
@@ -188,6 +191,30 @@ def _read_invlists(f, nlist_expected):
     return list_off, ids, rows, code_size
 
 
+# ------------------------------------------------------------------ PQ code packing
+def pack_codes(codes: np.ndarray, nbits: int) -> np.ndarray:
+    """codes [n, M] (one code per byte) -> rows of M * nbits / 8 bytes in faiss bit order."""
+    codes = np.ascontiguousarray(codes, dtype=np.uint8)
+    if nbits == 8:
+        return codes
+    if nbits != 4 or codes.shape[1] % 2:
+        raise FaissFormatError(f"cannot pack {codes.shape[1]} codes of {nbits} bits")
+    return (codes[:, 0::2] & 15) | ((codes[:, 1::2] & 15) << 4)
+
+
+def unpack_codes(rows: np.ndarray, M: int, nbits: int) -> np.ndarray:
+    """rows of M * nbits / 8 bytes in faiss bit order -> codes [n, M], one code per byte."""
+    rows = np.ascontiguousarray(rows, dtype=np.uint8).reshape(-1, M * nbits // 8)
+    if nbits == 8:
+        return rows
+    if nbits != 4:
+        raise FaissFormatError(f"cannot unpack codes of {nbits} bits")
+    out = np.empty((rows.shape[0], M), dtype=np.uint8)
+    out[:, 0::2] = rows & 15
+    out[:, 1::2] = rows >> 4
+    return out
+
+
 # ------------------------------------------------------------------ public
 def write_index(state: Dict, path: str, nprobe: int = 1) -> None:
     """state: engine / oracle `get_state()` dict.  Writes a faiss index file."""
@@ -202,16 +229,20 @@ def write_index(state: Dict, path: str, nprobe: int = 1) -> None:
             _write_invlists(f, state["list_off"], state["ids"], vecs, 4 * int(state["d"]))
         elif kind == "ivf_pq":
             M, ksub = int(state["M"]), int(state["ksub"])
-            if ksub != 256:
-                raise FaissFormatError("only 8-bit product quantizers are supported")
+            nbits = {256: 8, 16: 4}.get(ksub)
+            if nbits is None:
+                raise FaissFormatError("only 8-bit and 4-bit product quantizers are supported")
+            code_size = M * nbits // 8
             f.write(b"IwPQ")
             _write_ivf_header(f, state, METRIC_L2, int(state["coarse_metric"]), nprobe)
             _w(f, "B", 1)  # by_residual
-            _w(f, "Q", M)  # code_size
-            _w(f, "QQQ", int(state["d"]), M, 8)
+            _w(f, "Q", code_size)
+            _w(f, "QQQ", int(state["d"]), M, nbits)
             _wvec(f, state["codebooks"], np.float32)
             codes = np.ascontiguousarray(state["codes"], dtype=np.uint8)
-            _write_invlists(f, state["list_off"], state["ids"], codes, M)
+            if codes.ndim != 2 or codes.shape[1] != code_size:
+                raise FaissFormatError(f"IndexIVFPQ: codes must be [ntotal, {code_size}] bytes (M * nbits / 8)")
+            _write_invlists(f, state["list_off"], state["ids"], codes, code_size)
         elif kind == "ivf_sq":
             d = int(state["d"])
             f.write(b"IwSq")
@@ -250,13 +281,14 @@ def read_index(path: str) -> Tuple[Dict, int]:
             (code_size,) = _r(f, "Q")
             pd, M, nbits = _r(f, "QQQ")
             cb = _rvec(f, np.float32)
-            if not by_res or nbits != 8 or pd != d or code_size != M:
-                raise FaissFormatError("IndexIVFPQ: only by_residual, 8 bits per sub-quantizer is supported")
+            if not by_res or nbits not in (4, 8) or pd != d or code_size != M * nbits // 8:
+                raise FaissFormatError("IndexIVFPQ: only by_residual, 4 or 8 bits per sub-quantizer is supported")
             if metric != METRIC_L2:
                 raise FaissFormatError("IndexIVFPQ: only METRIC_L2 is supported")
             list_off, ids, rows, cs = _read_invlists(f, nlist)
-            st.update(kind="ivf_pq", coarse_metric=cmetric, M=M, ksub=256,
-                      codebooks=cb.reshape(M, 256, d // M), codes=rows.reshape(-1, M))
+            ksub = 1 << nbits
+            st.update(kind="ivf_pq", coarse_metric=cmetric, M=M, ksub=ksub,
+                      codebooks=cb.reshape(M, ksub, d // M), codes=rows.reshape(-1, code_size))
         else:
             qtype, _, _ = _r(f, "iif")
             sd, scs = _r(f, "QQ")

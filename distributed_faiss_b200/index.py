@@ -12,7 +12,8 @@ Builders (reference index.py:93-100):
   "flat"       -> IndexFlatIP            (always inner product, quirk B1 of SURVEY.md)
   "ivf_simple" -> IndexIVFFlat(metric)   nprobe = cfg.nprobe
   "knnlm"      -> IndexIVFPQ             always L2 / by_residual; M = extra["code_size"] (64),
-                                          nbits = extra["bits_per_vector"] (8); cfg.nprobe is
+                                          nbits = extra["bits_per_vector"] (8; 4 halves the
+                                          code bytes, needs M % 8 == 0); cfg.nprobe is
                                           overwritten by the index default 1 (quirk B3)
   "ivfsq"      -> IndexIVFScalarQuantizer(QT_fp16), always L2, nprobe = cfg.nprobe
 "hnswsq", "ivf_gpu" and free-form `faiss_factory` strings are outside the hot path this

@@ -53,7 +53,8 @@ typedef struct dfx_cfg {
                          index, which is therefore always L2 (index.py:44-46, 64-66). */
     int32_t d;        /* vector dimension (cfg.dim) */
     int32_t pq_m;     /* IVF_PQ: sub-quantizers  (cfg.extra["code_size"], index.py:44) */
-    int32_t pq_nbits; /* IVF_PQ: bits per code   (cfg.extra["bits_per_vector"], index.py:45) */
+    int32_t pq_nbits; /* IVF_PQ: bits per code, 8 or 4 (cfg.extra["bits_per_vector"], index.py:45);
+                         4 needs pq_m % 8 == 0 */
     int32_t device;   /* CUDA device ordinal this shard lives on */
     int64_t nlist;    /* IVF_*: number of inverted lists (cfg.centroids) */
 } dfx_cfg;
@@ -79,8 +80,9 @@ int dfx_add_dev(dfx_index *idx, int64_t n, const float *d_x, void *stream);
  *   "tc_auto_window" (16384): rows AUTO observes before PRECISE may become FAST;
  * "flat_tensor_cores" (1): 0 runs FLAT searches through the FFMA GEMM instead of the tensor-core
  *   screening + exact re-rank;
- * "interleaved" (1): 0 keeps IVF-PQ (M = 32) codes row-major (one vector per lane, table from
- *   pq_prep_kernel) instead of the block-interleaved layout of the fused table-build + scan;
+ * "interleaved" (1): 0 keeps IVF-PQ (M = 32 x 8 bit, M = 64 x 4 bit) codes row-major (one vector
+ *   per lane, table from pq_prep_kernel) instead of the block-interleaved layout of the fused
+ *   table-build + scan;
  * "il2_threads" (0 = 256) / "il2_prefetch" (-1 = 4 blocks): CTA shape and L2 prefetch distance of
  *   that scan (tuning);
  * "rows_inflight" (0 = by row size): 4 or 8 vectors per warp in flight in the IVF-Flat / IVF-SQ
@@ -167,7 +169,9 @@ int dfx_map_ids_dev(int64_t n, const int64_t *d_ids, const int64_t *d_table, int
 /* ---- state exchange (tests, persistence; not on the timed path) ----
  * named arrays, host memory, list-sorted storage order:
  *   "centroids" f32[nlist,d]   "codebooks" f32[M,ksub,dsub]   "list_off" i64[nlist+1]
- *   "ids" i64[ntotal]   "codes" u8[ntotal,M]   "tvals" f32[ntotal]
+ *   "ids" i64[ntotal]   "codes" u8[ntotal,M*nbits/8]   "tvals" f32[ntotal]
+ *   ("codes" in faiss bit order: at nbits = 4 code m is the low nibble of byte m/2 when m is
+ *   even, the high nibble when m is odd; ksub = 1 << nbits)
  *   "vecs" f32[ntotal,d] (IVF_FLAT)   "codes16" u16[ntotal,d]   "xb" f32[ntotal,d] (FLAT)
  * dfx_get_array with out == NULL only reports the size.  Import order: centroids,
  * codebooks, then list_off, ids and the payload, then dfx_import_done(). */
